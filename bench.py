@@ -21,6 +21,10 @@ configs[3], the configuration the metric is quoted on.
   roofline : integer-multiply pipe: executed MAC32 of the dominant kernel / its measured duration / measured peak.
   cpu_baseline : the C++ port of the reference algorithm (oracle/oracle.cpp) on the box's host cores, contribute +
           verify on a bounded sample, rank 0 at N = 1 only.
+
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last step returned to its caller as float32 /
+          float64 .npy files (see dump_outputs), so two builds can be compared output for output.  The inputs depend
+          only on the arguments, and the sample of elements is fixed by DUMP_SEED.
 """
 import argparse
 import hashlib
@@ -48,6 +52,9 @@ W_REF_POWER = 6109950
 W_EXEC_G1_MUL = 775 * 300 + 890 * 234
 W_EXEC_G2_MUL = 3200 * 300
 METRIC = "phase1 contribute+verify G1+G2 powers/sec at 2^22 (1/2/4/8 B200), bit-exact"
+VECTORS = ("tau_g1", "tau_g2", "alpha_g1", "beta_g1", "beta_g2")
+DUMP_SEED = 20261020
+DUMP_ELEMENTS = 8192  # per vector: 8192 x 720 B of response + new challenge = 24 MB as float32
 
 
 def derive_scalar(seed: bytes, label: bytes) -> int:
@@ -277,6 +284,45 @@ def run_extras(S, R, O, bw6_power, phase2_log2):
     return out
 
 
+def dump_sample(count, vector):
+    """Sorted element indices of `vector` that --dump-outputs writes: all of them up to DUMP_ELEMENTS, else a fixed
+    seeded sample."""
+    import numpy as np
+    if count <= DUMP_ELEMENTS:
+        return np.arange(count)
+    return np.sort(np.random.default_rng([DUMP_SEED, vector]).choice(count, DUMP_ELEMENTS, replace=False))
+
+
+def dump_outputs(out_dir, buffers, pairs, accepted, rank, world, dist=None):
+    """Writes what one round returns to its caller:
+      <buffer>_<vector>.npy  float32 [elements, element bytes]: the bytes of the dump_sample elements of each vector of
+                             every (buffer name, device uint8 tensor, sharding.vector_offsets) in `buffers`;
+      ratio_pairs.npy        float32 bytes of the (s, sx) blob the four ratio checks read (reduced over ranks);
+      verdict.npy            float64 [1]: 1 when the four checks accepted the response.
+    Each rank contributes the sampled elements of its own shard, so the files do not depend on the number of GPUs."""
+    import numpy as np
+    import torch
+    from snark_setup_b200 import sharding
+    arrays = {}
+    for v, name in enumerate(VECTORS):
+        for label, buf, offs in buffers:
+            o, cnt, sz = offs[v]
+            idx = torch.from_numpy(dump_sample(cnt, v)).to(buf.device)
+            rows = buf[o:o + cnt * sz].view(cnt, sz).index_select(0, idx).float()
+            s, e = sharding.shard_range(cnt, rank, world)
+            rows[(idx < s) | (idx >= e)] = 0  # computed by another rank
+            if world > 1:
+                dist.all_reduce(rows)
+            arrays[f"{label}_{name}"] = rows.cpu().numpy()
+    if rank != 0:
+        return
+    arrays["ratio_pairs"] = np.frombuffer(pairs, dtype=np.uint8).astype(np.float32)
+    arrays["verdict"] = np.array([1.0 if accepted else 0.0])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _STDOUT_FD = None
 _T0 = time.perf_counter()
 
@@ -310,8 +356,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the one-step C3 (BW6-761) / C5 (phase 2) measurements")
     ap.add_argument("--extras-bw6-power", type=int, default=21)
     ap.add_argument("--extras-phase2-log2", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's response, new challenge, ratio pairs and verdict to DIR/*.npy")
     ap.add_argument("--cpu-baseline-only", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.cpu_baseline_only:
         print(json.dumps(cpu_baseline()), flush=True)
         return
@@ -397,6 +447,7 @@ def main():
     nblob = S.pairs_size(cid)
     d_blob = torch.zeros(nblob, dtype=torch.uint8, device=dev)
     d_all = torch.zeros(nblob * world, dtype=torch.uint8, device=dev)
+    last_pairs = [None]  # rank 0: the whole (s, sx) blob of the latest verification
 
     def verdict(blob):
         """partial blob of this rank -> (gather) -> rank 0: sum + the four check_same_ratio.  Returns True / False / None."""
@@ -407,6 +458,7 @@ def main():
                 return None
             blob = S.phase1_reduce_partial_pairs(cid, [d_all[i * nblob:(i + 1) * nblob].cpu().numpy().tobytes()
                                                        for i in range(world)], raw=True)
+        last_pairs[0] = blob
         try:
             S.phase1_check_ratio_pairs(cid, blob, g1_check, g2_check)
             return True
@@ -446,6 +498,10 @@ def main():
     launches = ffi.profile_launches()
     value = N * args.steps / (dev_ms * 1e-3)
     verdict_ok = all(v is True for v in verdicts) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [("response", response, offs_c), ("new_challenge", newc, offs_u)], last_pairs[0],
+                     verdicts[-1], rank, world, dist)
+        progress("outputs of the last timed step written to %s" % args.dump_outputs)
 
     # per-kernel durations for the roofline: one extra round with the vectors SERIALISED on one stream, so the
     # event brackets around each launch measure that kernel alone (in the timed region above the five vectors
