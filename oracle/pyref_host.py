@@ -49,6 +49,45 @@ def chacha20_block(key: bytes, counter: int):
     return [(a + b) & 0xffffffff for a, b in zip(s, init)]
 
 
+def chacha20_blocks(key: bytes, first: int, n: int):
+    """chacha20_block for the counters first .. first + n - 1 at once (numpy, one lane per block) -> uint32 [n, 16].
+    The pure-Python block takes minutes over the 2^21 blocks of one MSM tile."""
+    import numpy as np
+    k = np.frombuffer(bytes(key), dtype="<u4")
+    ctr = np.arange(first, first + n, dtype=np.uint64)
+    consts = (0x61707865, 0x3320646e, 0x79622d32, 0x6b206574)
+    init = [np.full(n, c, np.uint32) for c in consts] + [np.full(n, w, np.uint32) for w in k]
+    init += [(ctr & 0xffffffff).astype(np.uint32), (ctr >> np.uint64(32)).astype(np.uint32), np.zeros(n, np.uint32),
+             np.zeros(n, np.uint32)]
+    x = [v.copy() for v in init]
+    t = np.empty(n, np.uint32)
+
+    def rotl(v, r):
+        np.right_shift(v, np.uint32(32 - r), out=t)
+        np.left_shift(v, np.uint32(r), out=v)
+        np.bitwise_or(v, t, out=v)
+
+    def qr(a, b, c, d):
+        for (p, q, s, r) in ((a, b, d, 16), (c, d, b, 12), (a, b, d, 8), (c, d, b, 7)):
+            np.add(x[p], x[q], out=x[p])
+            np.bitwise_xor(x[s], x[p], out=x[s])
+            rotl(x[s], r)
+
+    for _ in range(10):
+        qr(0, 4, 8, 12); qr(1, 5, 9, 13); qr(2, 6, 10, 14); qr(3, 7, 11, 15)
+        qr(0, 5, 10, 15); qr(1, 6, 11, 12); qr(2, 7, 8, 13); qr(3, 4, 9, 14)
+    for v, v0 in zip(x, init):
+        np.add(v, v0, out=v)
+    return np.stack(x, axis=1)
+
+
+def rho(seed: bytes, first: int, n: int):
+    """The random scalars of the device ratio-check MSM (snark-setup_b200/csrc/msm.cuh): rho_i = the first 16 bytes of
+    ChaCha20(key = seed, counter = first + i, nonce = 0) as a little-endian integer, for i < n."""
+    raw = chacha20_blocks(seed, first, n)[:, :4].astype("<u4").tobytes()
+    return [int.from_bytes(raw[16 * i:16 * i + 16], "little") for i in range(n)]
+
+
 class ChaChaRng:
     def __init__(self, seed32: bytes):
         assert len(seed32) == 32

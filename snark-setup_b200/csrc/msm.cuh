@@ -48,7 +48,7 @@ struct RhoSource {
     uint32_t key[8];               // ChaCha20 key when explicit_rho == nullptr
     uint64_t first_index;          // global index of element 0 (ChaCha counter base)
     int frw;                       // scalar words
-    int nbits;                     // scalar bits actually used (W*c >= 128 for generated, field bits for explicit)
+    int nbits;                     // scalar bits actually used (128 = W*c for generated, field bits for explicit)
 };
 
 // c-bit digit `w` of the scalar of element i

@@ -1,7 +1,8 @@
 """GPU tests at sizes the oracle cannot reach in seconds, through size-independent properties of the path
 (BASELINE.json configs): contribute is a group action, so contributing (tau, alpha, beta) and then their
 inverses must give back the original accumulator byte for byte; a verified response must satisfy
-sx = tau * s for every vector; decompress(compress(x)) = x; phase-2 batch_mul by delta then delta^-1 is the
+sx = tau * s for every vector, and its (s, sx) are the exact sums of the known discrete logs whether the round is
+verified whole or shard by shard; decompress(compress(x)) = x; phase-2 batch_mul by delta then delta^-1 is the
 identity.  Sizes: 2^18 powers by default; SS_TEST_FULL=1 runs BASELINE.json's own sizes — 2^22 BLS12-377 (configs[3], the
 metric's configuration) and 2^21 BW6-761 (configs[2]); logs under profiles/."""
 import hashlib
@@ -12,6 +13,7 @@ import pytest
 
 import coracle as O
 import pyref as R
+import pyref_host as H
 import snark_setup_b200 as S
 
 pytestmark = pytest.mark.gpu
@@ -56,10 +58,28 @@ def test_contribute_inverse_roundtrip_and_verify(curve, power):
             assert bytes(resp[oo + i0 * so:oo + (i0 + n) * so]) == want, (vec, i0)
     # verification of the response: new challenge + ratio pairs
     newc = bytearray(sp.get_length(False))
-    pairs = S.phase1_verification_vectors(sp, bytes(resp), True, newc, False, seed=hashlib.blake2b(b"rho", digest_size=32).digest())
+    seed = hashlib.blake2b(b"rho", digest_size=32).digest()
+    pairs = S.phase1_verification_vectors(sp, bytes(resp), True, newc, False, seed=seed)
     tau_acc = k0[0] * k1[0] % cv.r
     for (s_, sx), grp in zip(pairs, (0, 1, 0, 0)):
         assert O.apply_powers(cid, grp, s_, False, 3, False, 1, powers=[tau_acc]) == sx
+    # the exact pairs: element i of a vector is coef * t^i * G and rho_i is keyed by the vector-relative index, so
+    # (s, sx) = coef * (sum_i rho_i t^i) * (G, t * G) over the n - 1 pairs
+    coefs = (1, 1, k0[1] * k1[1], k0[2] * k1[2])
+    for vec, ((s_, sx), coef) in enumerate(zip(pairs, coefs)):
+        g = cv.g2 if vec == 1 else cv.g1
+        rho = H.rho(seed, 0, rp.split_offsets(True)[vec][1] - 1)
+        acc, t_i = 0, 1
+        for x in rho:
+            acc += x * t_i
+            t_i = t_i * tau_acc % cv.r
+        k = coef * acc % cv.r
+        assert (s_, sx) == (g.encode(g.mul(g.gen, k), False), g.encode(g.mul(g.gen, k * tau_acc % cv.r), False)), vec
+    # the same round verified shard by shard: the partial pairs add up to the same bytes
+    for world in ((4, 8) if FULL else (3, 8)):
+        blobs = [S.phase1_verification_vectors(sp, bytes(resp), True, None, False, seed=seed, shard=(r, world), raw=True)
+                 for r in range(world)]
+        assert S.phase1_reduce_partial_pairs(cid, blobs) == pairs, world
     # contribute the inverse keys on the new challenge: back to the first challenge, byte for byte
     back = bytearray(sp.get_length(False))
     S.phase1_computation(sp, bytes(newc), back, False, False, S.CHECK_NO, *k1inv)
