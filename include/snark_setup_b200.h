@@ -37,10 +37,13 @@ extern "C" {
 
 /* The curves the reference exposes (setup-utils/src/converters.rs:18-45).  BLS12-377 and BW6-761 are the tuned ceremony
  * curves.  MNT4-753 / MNT6-753 (a != 0, G2 over Fq2 / Fq3, 95-byte field elements) run the same entry points
- * functionally — batch_exp / apply_powers / Phase1::computation, transcode, subgroup checks, merge_pairs / power_pairs
- * and the verification vectors — without endomorphism speed-ups; not available for them: ss_phase1_initialization (the
- * arkworks G2 generator constants are not known to this build), the device pairing checks (ss_*same_ratio*; the (s, sx)
- * pairs are returned for the host's check_same_ratio as SURVEY.md §8 A12 places it), group FFT and QAP. */
+ * functionally — batch_exp / apply_powers / Phase1::computation, transcode, subgroup checks, merge_pairs / power_pairs,
+ * the verification vectors, and prepare_phase2 / QAP evaluation (ss_group_ifft, ss_h_query_groth16,
+ * ss_groth16_params_*, ss_qap_dot_product) — without endomorphism speed-ups.  Their radix-2 domains reach 2^30 (MNT4-753
+ * Fr) and 2^15 (MNT6-753 Fr); a larger domain fails with SS_ERR_INVALID_ARGUMENT.  Not available for them:
+ * ss_phase1_initialization (the arkworks G2 generator constants are not known to this build) and the device pairing
+ * checks (ss_*same_ratio*; the (s, sx) pairs are returned for the host's check_same_ratio as SURVEY.md §8 A12 places
+ * it). */
 typedef enum { SS_CURVE_BLS12_377 = 0, SS_CURVE_BW6_761 = 1, SS_CURVE_MNT4_753 = 2, SS_CURVE_MNT6_753 = 3 } ss_curve;
 typedef enum { SS_G1 = 0, SS_G2 = 1 } ss_group;
 
@@ -307,7 +310,8 @@ int ss_h_query_groth16(int curve, const uint8_t* powers, int in_compressed, int 
 
 /* domain_size (groth16_utils.rs:65-69) and the byte length Groth16Params::write produces
  * (groth16_utils.rs:134-168): alpha_g1, beta_g1, beta_g2, coeffs_g1[m], coeffs_g2[m],
- * alpha_coeffs_g1[m], beta_coeffs_g1[m], h_g1[m-1]. */
+ * alpha_coeffs_g1[m], beta_coeffs_g1[m], h_g1[m-1].  m above 2^(2-adicity of Fr) has no radix-2 domain =>
+ * SS_ERR_INVALID_ARGUMENT (only MNT6-753, 2-adicity 15, reaches that at practical sizes). */
 int ss_groth16_params_size(int curve, uint64_t phase2_size, int compressed, uint64_t* domain_size, size_t* bytes);
 
 /* Groth16Params::new + ::write — setup-utils/src/groth16_utils.rs:81-131,134-168, the body of

@@ -163,5 +163,9 @@ const FftOps& fft_ops_bls377_g1();
 const FftOps& fft_ops_bls377_g2();
 const FftOps& fft_ops_bw6_g1();
 const FftOps& fft_ops_bw6_g2();
+const FftOps& fft_ops_mnt4_g1();
+const FftOps& fft_ops_mnt4_g2();
+const FftOps& fft_ops_mnt6_g1();
+const FftOps& fft_ops_mnt6_g2();
 
 }  // namespace ss

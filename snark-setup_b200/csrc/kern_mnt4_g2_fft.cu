@@ -1,0 +1,16 @@
+// Group-FFT and QAP kernel instantiations for Mnt4G2 (coordinates over Fq2): k_fft_butterfly, k_h_query and the
+// QAP sums of fft.cuh / qap.cuh.  The twiddle and coefficient multiplications run on k_scalar_mul of kern_mnt4_g2.cu
+// (double-and-add, no endomorphism).  The exceptional P = Q case of the additions doubles through jac_dbl_cold, which
+// takes the a != 0 formula (CurveCoeffA in ec.cuh).  A translation unit of its own keeps nvcc compile times parallel.
+#include "qap.cuh"
+
+namespace ss {
+const FftOps& fft_ops_mnt4_g2() {
+    static const FftOps o = FftLaunch<Mnt4G2>::ops();
+    return o;
+}
+const QapOps& qap_ops_mnt4_g2() {
+    static const QapOps o = QapLaunch<Mnt4G2>::ops();
+    return o;
+}
+}  // namespace ss

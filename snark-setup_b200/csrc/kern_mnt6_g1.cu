@@ -1,6 +1,6 @@
 // Kernel instantiations for Mnt6G1 (MNT4/6-753 are exposed by the reference, setup-utils/src/converters.rs:18-45): the
 // generic kernels over a 24-limb field with a != 0 formulas and byte-granular serialisation.  Functional coverage, not
-// a tuned path: no endomorphism, no group FFT / QAP / pairing instantiations.
+// a tuned path: no endomorphism, no pairing instantiations; the group-FFT / QAP kernels are in kern_mnt6_g1_fft.cu.
 #include "msm.cuh"
 
 namespace ss {

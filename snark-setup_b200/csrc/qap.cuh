@@ -78,5 +78,9 @@ const QapOps& qap_ops_bls377_g1();
 const QapOps& qap_ops_bls377_g2();
 const QapOps& qap_ops_bw6_g1();
 const QapOps& qap_ops_bw6_g2();
+const QapOps& qap_ops_mnt4_g1();
+const QapOps& qap_ops_mnt4_g2();
+const QapOps& qap_ops_mnt6_g1();
+const QapOps& qap_ops_mnt6_g2();
 
 }  // namespace ss
