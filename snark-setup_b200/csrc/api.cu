@@ -4,7 +4,7 @@
 //   Phase1Parameters::new / chunk_sizes   phase1/src/objects/parameters.rs:115-294
 //   split / split_mut                     phase1/src/helpers/buffers.rs:246-341
 //   apply_powers                          phase1/src/helpers/buffers.rs:77-97
-//   Phase1::computation (Groth16)         phase1/src/computation.rs:40-193
+//   Phase1::computation                   phase1/src/computation.rs:40-302
 // The reference walks each vector in `batch_size` windows on rayon threads; results do not depend
 // on the windowing, so here each vector is cut into device tiles (default 1 212 416 elements) that are
 // pipelined over two CUDA streams (H2D of tile k+1 overlaps the kernels of tile k), the five vectors
@@ -533,109 +533,127 @@ void part_range(uint64_t n, uint64_t part, uint64_t parts, uint64_t* s0, uint64_
     *e0 = *s0 + base + (part < rem ? 1 : 0);
 }
 
-// Marlin's short tau_g2 / alpha_g1 vectors live in the buffer of chunk_index 0 — the ONE predicate the reference uses for
-// the sizes (parameters.rs:152-160), the buffer split (buffers.rs:151,220,274,324) and the computation
-// (computation.rs:198); full-mode callers pass chunk_index = 0.  Sizes, computation, verification and
-// initialization here all go through this function so they cannot disagree about the buffer layout.
-bool is_chunk0(const ss_phase1_params* p) { return p->chunk_index == 0; }
+// Runs job(0) .. job(n - 1) and returns the first failure.  When n == 1 or !parallel the jobs run in order on the
+// calling thread and stop at the first failure; otherwise each gets a thread of its own.  g_err is thread-local, so a
+// failing thread's record is copied out, and after the join the lowest-indexed failure is restored and returned.
+template <class F>
+int run_jobs(int n, bool parallel, F job) {
+    if (n == 1 || !parallel) {
+        for (int i = 0; i < n; i++)
+            if (int rc = job(i)) return rc;
+        return SS_OK;
+    }
+    std::vector<int> rcs(n, SS_OK);
+    std::vector<ss_error_info> errs(n);
+    std::vector<std::thread> th;
+    for (int i = 0; i < n; i++)
+        th.emplace_back([&, i] {
+            if ((rcs[i] = job(i))) errs[i] = g_err;
+        });
+    for (auto& t : th) t.join();
+    for (int i = 0; i < n; i++)
+        if (rcs[i]) {
+            g_err = errs[i];
+            return rcs[i];
+        }
+    return SS_OK;
+}
 
-int phase1_sizes(const ss_phase1_params* p, ss_phase1_sizes* o) {
-    if (!p || !o) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "null argument");
+// The five vectors of a phase-1 buffer, in buffer order, with their groups
+const int kVecGroup[5] = {SS_G1, SS_G2, SS_G1, SS_G1, SS_G2};
+const char* const kVecName[5] = {"tau_g1", "tau_g2", "alpha_g1", "beta_g1", "beta_g2"};
+
+// The phase-1 buffer of one chunk, split / split_mut (buffers.rs:246-341): the 64-byte hash, then
+// [tau_g1][tau_g2][alpha_g1][beta_g1][beta_g2].  Marlin has tau_g1 and, in the buffer of chunk 0 only, k+2 tau_g2 and
+// 3+3k alpha_g1 elements; its beta counts are zero.  Phase1Parameters::new / chunk_sizes (parameters.rs:115-294) give
+// the counts.
+struct Phase1Layout {
+    uint64_t powers_length, powers_g1_length, g1_chunk_size, other_chunk_size;
+    struct Vector {
+        const GroupOps* ops;
+        int group;
+        uint64_t size, count, off;  // bytes per element, elements, byte offset in the buffer
+        const char* name;
+    } v[5];
+    uint64_t end;  // bytes of the buffer, without the public key
+};
+
+int phase1_layout(const ss_phase1_params* p, int compressed, Phase1Layout* L) {
+    if (!p) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "null argument");
     const GroupOps* g1 = group_ops(p->curve, SS_G1);
     const GroupOps* g2 = group_ops(p->curve, SS_G2);
     if (!g1 || !g2) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "unknown curve %d", p->curve);
     if (p->total_size_in_log2 == 0 || p->total_size_in_log2 > 40)
         return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "bad power %u", p->total_size_in_log2);
-    const uint64_t pl = 1ull << p->total_size_in_log2, pg1 = (pl << 1) - 1;
-    const uint64_t upper = p->proving_system == SS_GROTH16 ? pg1 : pl;
+    const bool groth16 = p->proving_system == SS_GROTH16;
+    const uint64_t k = p->total_size_in_log2, pl = 1ull << k, pg1 = (pl << 1) - 1;
+    const uint64_t upper = groth16 ? pg1 : pl;
     uint64_t start = 0, end = upper;
     if (p->contribution_mode == SS_MODE_CHUNKED) {
         start = p->chunk_index * p->chunk_size;
         end = (p->chunk_index + 1) * p->chunk_size;
         if (p->chunk_size == 0 || start >= upper) return fail(SS_ERR_INVALID_CHUNK, 0, 0, 0, "chunk out of range");
     }
-    o->powers_length = pl;
-    o->powers_g1_length = pg1;
-    o->g1_chunk_size = end > upper ? upper - start : end - start;
-    if (p->proving_system == SS_GROTH16) {
-        if (end > pl && start >= pl) o->other_chunk_size = 0;
-        else if (end > pl) o->other_chunk_size = pl - start;
-        else o->other_chunk_size = end - start;
-    } else {
-        o->other_chunk_size = 0;
+    L->powers_length = pl;
+    L->powers_g1_length = pg1;
+    L->g1_chunk_size = std::min(end, upper) - start;
+    L->other_chunk_size = groth16 && start < pl ? std::min(end, pl) - start : 0;
+    // Marlin's short tau_g2 / alpha_g1 vectors live in the buffer of chunk_index 0 — the ONE predicate the reference
+    // uses for the sizes (parameters.rs:152-160), the buffer split (buffers.rs:151,220,274,324) and the computation
+    // (computation.rs:198); full-mode callers pass chunk_index = 0.
+    const bool chunk0 = p->chunk_index == 0;
+    const uint64_t n2 = L->other_chunk_size;
+    const uint64_t cnt[5] = {L->g1_chunk_size, groth16 ? n2 : (chunk0 ? k + 2 : 0), groth16 ? n2 : (chunk0 ? 3 + 3 * k : 0),
+                             groth16 ? n2 : 0, groth16 ? 1u : 0u};
+    uint64_t off = 64;
+    for (int v = 0; v < 5; v++) {
+        Phase1Layout::Vector& e = L->v[v];
+        e.group = kVecGroup[v];
+        e.ops = e.group == SS_G1 ? g1 : g2;
+        e.size = compressed ? e.ops->csize : e.ops->usize;
+        e.count = cnt[v];
+        e.off = off;
+        e.name = kVecName[v];
+        off += e.count * e.size;
     }
-    o->hash_size = 64;
-    o->public_key_size = 3 * (uint64_t)g2->csize + 6 * (uint64_t)g1->csize;
-    const uint64_t k = p->total_size_in_log2;
-    if (p->proving_system == SS_GROTH16) {
-        o->accumulator_size = o->g1_chunk_size * g1->usize + o->other_chunk_size * (g2->usize + 2 * (uint64_t)g1->usize) + g2->usize + 64;
-        o->contribution_size = o->g1_chunk_size * g1->csize + o->other_chunk_size * (g2->csize + 2 * (uint64_t)g1->csize) + g2->csize + 64 + o->public_key_size;
-    } else {
-        uint64_t xu = 0, xc = 0;
-        if (is_chunk0(p)) {
-            xu = 3 * (uint64_t)g1->usize + 3 * k * g1->usize + (k + 2) * g2->usize;
-            xc = 3 * (uint64_t)g1->csize + 3 * k * g1->csize + (k + 2) * g2->csize;
-        }
-        o->accumulator_size = o->g1_chunk_size * g1->usize + xu + 64;
-        o->contribution_size = o->g1_chunk_size * g1->csize + xc + 64 + o->public_key_size;
-    }
+    L->end = off;
     return SS_OK;
 }
 
-// Phase1::computation, Marlin branch (phase1/src/computation.rs:195-302): tau_g1 over the chunk's powers as in
-// Groth16; on chunk 0 additionally the k+2 tau_g2 and 3+3k alpha_g1 elements, whose scalars (inverse degree-bound
-// powers etc.) are produced by k_marlin_scalars and applied through the explicit-exponent path.
-int phase1_computation_marlin(const ss_phase1_params* p, const ss_phase1_sizes& z, const GroupOps& g1, const GroupOps& g2,
-                              const uint8_t* input, size_t input_len, uint8_t* output, size_t output_len, int cin, int cout,
-                              int check, const uint8_t* tau, const uint8_t* alpha, bool host, cudaStream_t user_stream,
-                              uint32_t shard_index, uint32_t shard_count) {
-    const uint64_t need_in = cin ? z.contribution_size - z.public_key_size : z.accumulator_size;
-    const uint64_t need_out = cout ? z.contribution_size - z.public_key_size : z.accumulator_size;
-    if (input_len < need_in) return fail(SS_ERR_INVALID_LENGTH, 0, need_in, input_len, "input buffer too short");
-    if (output_len < need_out) return fail(SS_ERR_INVALID_LENGTH, 0, need_out, output_len, "output buffer too short");
-    for (const uint8_t* s : {tau, alpha})
-        if (!scalar_is_canonical(p->curve, s)) return fail(SS_ERR_INVALID_DATA, 0, 0, 0, "scalar >= r");
-    int rc = ensure_init();
-    if (rc) return rc;
-    const int device = g_devices[0];
-    CU(cudaSetDevice(device));
-    const uint64_t k = p->total_size_in_log2;
-    const bool chunk0 = is_chunk0(p);
-    const uint64_t n_g2 = chunk0 ? k + 2 : 0, n_al = chunk0 ? 3 + 3 * k : 0;
-    auto sz = [&](const GroupOps& g, int c) { return (uint64_t)(c ? g.csize : g.usize); };
-    LaneGuard lane;
-    if ((rc = lane_acquire(device, 4096 + (n_g2 + n_al) * scalar_stride(g1), &lane.l))) return rc;
-    ScalarSetup sc;
-    const uint8_t* coeffs[3] = {nullptr, alpha, nullptr};
-    if ((rc = sc.init(g1, tau, coeffs, lane.l->stream))) return rc;
-    const uint64_t first = p->contribution_mode == SS_MODE_CHUNKED ? p->chunk_index * p->chunk_size : 0;
-    const uint64_t n1 = z.g1_chunk_size;
-    // index-range shard of tau_g1 (the short tau_g2 / alpha_g1 vectors belong to shard 0)
-    uint64_t s0, e0;
-    part_range(n1, shard_index, shard_count, &s0, &e0);
-    VectorJob jt = {&g1, input + 64 + s0 * sz(g1, cin), output + 64 + s0 * sz(g1, cout), cin, cout, check, e0 - s0, nullptr,
-                    sc.d_tab, first + s0, sc.d_coeff_m[0], 0, "tau_g1"};
-    if ((rc = run_vector_on(device, jt, host, user_stream))) {
-        g_err.index += s0;
-        return rc;
-    }
-    if (!chunk0 || shard_index != 0) return SS_OK;
-    uint8_t* d_g2s = lane.l->buf;
-    uint8_t* d_als = d_g2s + align_up(n_g2 * scalar_stride(g1), 256);
-    g1.marlin_scalars(sc.d_tab, z.powers_length, (int)k, reinterpret_cast<uint32_t*>(d_g2s), reinterpret_cast<uint32_t*>(d_als),
-                      lane.l->stream);
-    CU(cudaGetLastError());
-    CU(cudaStreamSynchronize(lane.l->stream));
-    const uint64_t oi2 = 64 + n1 * sz(g1, cin), oo2 = 64 + n1 * sz(g1, cout);
-    VectorJob j2 = {&g2, input + oi2, output + oo2, cin, cout, check, n_g2, d_g2s, sc.d_tab, 0, sc.d_coeff_m[0], 0, "tau_g2"};
-    j2.exps_on_device = true;
-    if ((rc = run_vector_on(device, j2, host, user_stream))) return rc;
-    const uint64_t oi3 = oi2 + n_g2 * sz(g2, cin), oo3 = oo2 + n_g2 * sz(g2, cout);
-    VectorJob j3 = {&g1, input + oi3, output + oo3, cin, cout, check, n_al, d_als, sc.d_tab, 0, sc.d_coeff_m[1], 1, "alpha_g1"};
-    j3.exps_on_device = true;
-    return run_vector_on(device, j3, host, user_stream);
+// SS_ERR_INVALID_LENGTH unless `len` bytes hold the buffer of layout `L`
+int check_length(const Phase1Layout& L, uint64_t len, const char* what) {
+    return len < L.end ? fail(SS_ERR_INVALID_LENGTH, 0, L.end, len, "%s", what) : SS_OK;
 }
 
+// The (s, sx) pairs blob of the four ratio-checked vectors: slot v holds s || sx of vector v, uncompressed, so
+// 4 x (s || sx) in the order G1, G2, G1, G1.  pair_slot(curve, 4) is the size of the blob, 0 for an unknown curve.
+size_t pair_slot(int curve, int v) {
+    size_t off = 0;
+    for (int u = 0; u < v; u++) {
+        const GroupOps* o = group_ops(curve, kVecGroup[u]);
+        if (!o) return 0;
+        off += 2 * (size_t)o->usize;
+    }
+    return off;
+}
+
+int phase1_sizes(const ss_phase1_params* p, ss_phase1_sizes* o) {
+    if (!p || !o) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "null argument");
+    Phase1Layout u, c;
+    int rc;
+    if ((rc = phase1_layout(p, 0, &u)) || (rc = phase1_layout(p, 1, &c))) return rc;
+    o->powers_length = u.powers_length;
+    o->powers_g1_length = u.powers_g1_length;
+    o->g1_chunk_size = u.g1_chunk_size;
+    o->other_chunk_size = u.other_chunk_size;
+    o->hash_size = 64;
+    o->public_key_size = 3 * (uint64_t)u.v[1].ops->csize + 6 * (uint64_t)u.v[0].ops->csize;
+    o->accumulator_size = u.end;
+    o->contribution_size = c.end + o->public_key_size;
+    return SS_OK;
+}
+
+// Phase1::computation (phase1/src/computation.rs:40-302), Groth16 and Marlin
 int phase1_computation_impl(const ss_phase1_params* p, const uint8_t* input, size_t input_len, uint8_t* output,
                             size_t output_len, int cin, int cout, int check, const uint8_t* tau,
                             const uint8_t* alpha, const uint8_t* beta, bool host, cudaStream_t user_stream,
@@ -645,38 +663,19 @@ int phase1_computation_impl(const ss_phase1_params* p, const uint8_t* input, siz
     if (shard_count == 0 || shard_index >= shard_count)
         return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "shard %u of %u", shard_index, shard_count);
     if (check < 0 || check > 3) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "bad check mode %d", check);
-    ss_phase1_sizes z;
-    int rc = phase1_sizes(p, &z);
-    if (rc) return rc;
-    const GroupOps& g1 = *group_ops(p->curve, SS_G1);
-    const GroupOps& g2 = *group_ops(p->curve, SS_G2);
-    if (p->proving_system == SS_MARLIN)
-        return phase1_computation_marlin(p, z, g1, g2, input, input_len, output, output_len, cin, cout, check, tau, alpha, host,
-                                         user_stream, shard_index, shard_count);
-    const uint64_t need_in = cin ? z.contribution_size - z.public_key_size : z.accumulator_size;
-    const uint64_t need_out = cout ? z.contribution_size - z.public_key_size : z.accumulator_size;
-    if (input_len < need_in) return fail(SS_ERR_INVALID_LENGTH, 0, need_in, input_len, "input buffer too short");
-    if (output_len < need_out) return fail(SS_ERR_INVALID_LENGTH, 0, need_out, output_len, "output buffer too short");
+    Phase1Layout li, lo;  // input, output
+    int rc;
+    if ((rc = phase1_layout(p, cin, &li)) || (rc = phase1_layout(p, cout, &lo))) return rc;
+    if ((rc = check_length(li, input_len, "input buffer too short"))) return rc;
+    if ((rc = check_length(lo, output_len, "output buffer too short"))) return rc;
+    const bool marlin = p->proving_system == SS_MARLIN;
+    if (marlin) beta = nullptr;  // Marlin has no beta
     for (const uint8_t* s : {tau, alpha, beta})
-        if (!scalar_is_canonical(p->curve, s)) return fail(SS_ERR_INVALID_DATA, 0, 0, 0, "scalar >= r");
+        if (s && !scalar_is_canonical(p->curve, s)) return fail(SS_ERR_INVALID_DATA, 0, 0, 0, "scalar >= r");
     if ((rc = ensure_init())) return rc;
-    // split (buffers.rs:293-341): [hash][tau_g1][tau_g2][alpha_g1][beta_g1][beta_g2]
-    auto sz = [&](const GroupOps& g, int c) { return (uint64_t)(c ? g.csize : g.usize); };
-    const uint64_t n1 = z.g1_chunk_size, n2 = z.other_chunk_size;
-    const uint64_t cnt[5] = {n1, n2, n2, n2, 1};
-    const GroupOps* gs[5] = {&g1, &g2, &g1, &g1, &g2};
-    const char* names[5] = {"tau_g1", "tau_g2", "alpha_g1", "beta_g1", "beta_g2"};
-    uint64_t oi[5], oo[5];
-    {
-        uint64_t a = 64, b = 64;
-        for (int v = 0; v < 5; v++) {
-            oi[v] = a;
-            oo[v] = b;
-            a += cnt[v] * sz(*gs[v], cin);
-            b += cnt[v] * sz(*gs[v], cout);
-        }
-    }
+    const GroupOps& g1 = *li.v[0].ops;
     const uint64_t first = p->contribution_mode == SS_MODE_CHUNKED ? p->chunk_index * p->chunk_size : 0;
+    const bool concurrent = concurrent_vectors();
 
     // One worker per device.  Every vector is cut into shard_count * D equal contiguous parts (SURVEY.md §8e:
     // balance by work, not by index — indices >= 2^k only carry one G1 element); this call owns parts
@@ -684,74 +683,51 @@ int phase1_computation_impl(const ss_phase1_params* p, const uint8_t* input, siz
     // because each part passes its own first power.  No inter-device / inter-process traffic.
     const int D = host ? (int)g_devices.size() : 1;
     const uint64_t parts = (uint64_t)shard_count * D;
-    auto worker = [&](int di, ss_error_info* err) -> int {
+    return run_jobs(D, true, [&](int di) -> int {
         const int device = host ? g_devices[di] : g_devices[0];
-        auto run = [&]() -> int {
-            CU(cudaSetDevice(device));
-            LaneGuard setup_lane;
-            int r = lane_acquire(device, 4096, &setup_lane.l);
-            if (r) return r;
-            ScalarSetup sc;
-            const uint8_t* coeffs[3] = {nullptr, alpha, beta};
-            if ((r = sc.init(g1, tau, coeffs, setup_lane.l->stream))) return r;
-            const uint32_t* cm[5] = {sc.d_coeff_m[0], sc.d_coeff_m[0], sc.d_coeff_m[1], sc.d_coeff_m[2], sc.d_coeff_m[2]};
-            const int hc[5] = {0, 0, 1, 1, 1};
-            // The five vectors run CONCURRENTLY, one host thread + lane (stream, scratch) each: the
-            // low-occupancy tails (batch normalisation, the single beta_g2 element) of one vector overlap the
-            // scalar multiplications of another.  SS_CONCURRENT_VECTORS=0 restores the sequential order.
-            auto one_vector = [&](int v) -> int {
-                uint64_t s0 = 0, e0 = cnt[v];
-                if (v == 4) {
-                    // beta_g2 <- beta * beta_g2 (computation.rs:42-50): tau^0 * beta, by the owner of part 0
-                    if (di != 0 || shard_index != 0) return SS_OK;
-                } else {
-                    part_range(cnt[v], (uint64_t)shard_index * D + di, parts, &s0, &e0);
-                }
-                VectorJob job = {gs[v], input + oi[v] + s0 * sz(*gs[v], cin), output + oo[v] + s0 * sz(*gs[v], cout), cin,
-                                 cout, check, e0 - s0, nullptr, sc.d_tab, v == 4 ? 0 : first + s0, cm[v], hc[v], names[v]};
-                int rv = run_vector_on(device, job, host, concurrent_vectors() ? nullptr : user_stream);
-                if (rv) g_err.index += s0;  // report vector-relative indices
-                return rv;
-            };
-            if (!concurrent_vectors()) {
-                for (int v = 0; v < 5; v++)
-                    if ((r = one_vector(v))) return r;
-                return SS_OK;
-            }
-            if (user_stream) CU(cudaStreamSynchronize(user_stream));  // work enqueued before the call comes first
-            int rv[5] = {0, 0, 0, 0, 0};
-            ss_error_info ev[5];
-            std::vector<std::thread> vt;
-            for (int v = 0; v < 5; v++)
-                vt.emplace_back([&, v] {
-                    cudaSetDevice(device);
-                    rv[v] = one_vector(v);
-                    if (rv[v]) ev[v] = g_err;
-                });
-            for (auto& t : vt) t.join();
-            for (int v = 0; v < 5; v++)
-                if (rv[v]) {
-                    g_err = ev[v];
-                    return rv[v];
-                }
-            return SS_OK;
-        };
-        int r = run();
-        if (r && err) *err = g_err;
-        return r;
-    };
-    if (D == 1) return worker(0, nullptr);
-    std::vector<std::thread> th;
-    std::vector<int> rcs(D, SS_OK);
-    std::vector<ss_error_info> errs(D);
-    for (int di = 0; di < D; di++) th.emplace_back([&, di] { rcs[di] = worker(di, &errs[di]); });
-    for (auto& t : th) t.join();
-    for (int di = 0; di < D; di++)
-        if (rcs[di]) {
-            g_err = errs[di];
-            return rcs[di];
+        CU(cudaSetDevice(device));
+        // beta_g2 <- beta * beta_g2 (computation.rs:42-50) and Marlin's tau_g2 / alpha_g1 are not split: the owner of
+        // part 0 does them whole.  The scalars of Marlin's two (computation.rs:195-302: inverse degree-bound powers
+        // etc.) are produced by k_marlin_scalars and applied through the explicit-exponent path.
+        const bool part0 = di == 0 && shard_index == 0;
+        const uint64_t n_g2 = part0 && marlin ? li.v[1].count : 0, n_al = part0 && marlin ? li.v[2].count : 0;
+        LaneGuard setup_lane;
+        int r = lane_acquire(device, 4096 + (n_g2 + n_al) * scalar_stride(g1), &setup_lane.l);
+        if (r) return r;
+        ScalarSetup sc;
+        const uint8_t* coeffs[3] = {nullptr, alpha, beta};
+        if ((r = sc.init(g1, tau, coeffs, setup_lane.l->stream))) return r;
+        uint8_t *d_g2s = nullptr, *d_als = nullptr;
+        if (n_g2 + n_al) {
+            d_g2s = setup_lane.l->buf;
+            d_als = d_g2s + align_up(n_g2 * scalar_stride(g1), 256);
+            g1.marlin_scalars(sc.d_tab, li.powers_length, (int)p->total_size_in_log2, reinterpret_cast<uint32_t*>(d_g2s),
+                              reinterpret_cast<uint32_t*>(d_als), setup_lane.l->stream);
+            CU(cudaGetLastError());
+            CU(cudaStreamSynchronize(setup_lane.l->stream));
         }
-    return SS_OK;
+        const uint8_t* exps[5] = {nullptr, d_g2s, d_als, nullptr, nullptr};
+        const uint32_t* cm[5] = {sc.d_coeff_m[0], sc.d_coeff_m[0], sc.d_coeff_m[1], sc.d_coeff_m[2], sc.d_coeff_m[2]};
+        const int hc[5] = {0, 0, 1, 1, 1};
+        // The five vectors run CONCURRENTLY, one host thread + lane (stream, scratch) each: the
+        // low-occupancy tails (batch normalisation, the single beta_g2 element) of one vector overlap the
+        // scalar multiplications of another.  SS_CONCURRENT_VECTORS=0 restores the sequential order.
+        auto one_vector = [&](int v) -> int {
+            cudaSetDevice(device);
+            const Phase1Layout::Vector &vi = li.v[v], &vo = lo.v[v];
+            const bool split = v == 0 || (!marlin && v < 4);  // powers of tau: split into parts
+            uint64_t s0 = 0, e0 = vi.count;
+            if (split) part_range(vi.count, (uint64_t)shard_index * D + di, parts, &s0, &e0);
+            else if (!part0) return SS_OK;
+            VectorJob job = {vi.ops, input + vi.off + s0 * vi.size, output + vo.off + s0 * vo.size, cin, cout, check,
+                             e0 - s0, exps[v], sc.d_tab, split ? first + s0 : 0, cm[v], hc[v], vi.name, true};
+            int rv = run_vector_on(device, job, host, concurrent ? nullptr : user_stream);
+            if (rv) g_err.index += s0;  // report vector-relative indices
+            return rv;
+        };
+        if (concurrent && user_stream) CU(cudaStreamSynchronize(user_stream));  // work enqueued before the call comes first
+        return run_jobs(5, concurrent, one_vector);
+    });
 }
 
 }  // namespace
@@ -996,25 +972,12 @@ int ss_check_subgroup(int curve, int group, const uint8_t* in, int compressed, s
 // source / destination offsets (phase1/src/aggregation.rs:11-180,189-353; helpers/accumulator.rs:182-301).
 static int copy_vectors(int curve, const uint8_t* src, const uint64_t* so, int src_c, uint8_t* dst, const uint64_t* dof,
                         int dst_c, const uint64_t* cnt, int check) {
-    const int grp[5] = {SS_G1, SS_G2, SS_G1, SS_G1, SS_G2};
     for (int v = 0; v < 5; v++) {
         if (!cnt[v]) continue;
-        int rc = transcode_impl(curve, grp[v], src + so[v], src_c, check, dst + dof[v], dst_c, cnt[v], false);
+        int rc = transcode_impl(curve, kVecGroup[v], src + so[v], src_c, check, dst + dof[v], dst_c, cnt[v], false);
         if (rc) return rc;
     }
     return SS_OK;
-}
-
-// byte offsets of the five vectors in a buffer laid out for `z` (buffers.rs:293-341)
-static void vector_offsets(int curve, const ss_phase1_sizes& z, int compressed, uint64_t* off) {
-    const GroupOps& g1 = *group_ops(curve, SS_G1);
-    const GroupOps& g2 = *group_ops(curve, SS_G2);
-    const uint64_t s1 = compressed ? g1.csize : g1.usize, s2 = compressed ? g2.csize : g2.usize;
-    off[0] = 64;
-    off[1] = off[0] + z.g1_chunk_size * s1;
-    off[2] = off[1] + z.other_chunk_size * s2;
-    off[3] = off[2] + z.other_chunk_size * s1;
-    off[4] = off[3] + z.other_chunk_size * s1;
 }
 
 static int chunk_vs_full(const ss_phase1_params* cp, int compressed_chunk, int compressed_full, size_t chunk_len, size_t full_len,
@@ -1025,27 +988,18 @@ static int chunk_vs_full(const ss_phase1_params* cp, int compressed_chunk, int c
     ss_phase1_params fp = *cp;
     fp.contribution_mode = SS_MODE_FULL;
     fp.chunk_index = 0;
-    ss_phase1_sizes cz, fz;
-    int rc = phase1_sizes(cp, &cz);
-    if (rc) return rc;
-    if ((rc = phase1_sizes(&fp, &fz))) return rc;
-    const GroupOps& g1 = *group_ops(cp->curve, SS_G1);
-    const GroupOps& g2 = *group_ops(cp->curve, SS_G2);
-    const uint64_t need_c = compressed_chunk ? cz.contribution_size - cz.public_key_size : cz.accumulator_size;
-    const uint64_t need_f = compressed_full ? fz.contribution_size - fz.public_key_size : fz.accumulator_size;
-    if (chunk_len < need_c) return fail(SS_ERR_INVALID_LENGTH, 0, need_c, chunk_len, "chunk buffer too short");
-    if (full_len < need_f) return fail(SS_ERR_INVALID_LENGTH, 0, need_f, full_len, "full buffer too short");
-    vector_offsets(cp->curve, cz, compressed_chunk, coff);
-    vector_offsets(cp->curve, fz, compressed_full, foff);
+    Phase1Layout c, f;
+    int rc;
+    if ((rc = phase1_layout(cp, compressed_chunk, &c)) || (rc = phase1_layout(&fp, compressed_full, &f))) return rc;
+    if ((rc = check_length(c, chunk_len, "chunk buffer too short"))) return rc;
+    if ((rc = check_length(f, full_len, "full buffer too short"))) return rc;
     // split_at_chunk(_mut): the chunk starts chunk_index * chunk_size elements into every vector
     const uint64_t first = cp->chunk_index * cp->chunk_size;
-    const uint64_t s1 = compressed_full ? g1.csize : g1.usize, s2 = compressed_full ? g2.csize : g2.usize;
-    foff[0] += first * s1;
-    foff[1] += first * s2;
-    foff[2] += first * s1;
-    foff[3] += first * s1;
-    cnt[0] = cz.g1_chunk_size;
-    cnt[1] = cnt[2] = cnt[3] = cz.other_chunk_size;
+    for (int v = 0; v < 5; v++) {
+        coff[v] = c.v[v].off;
+        foff[v] = f.v[v].off + (v < 4 ? first * f.v[v].size : 0);
+        cnt[v] = c.v[v].count;
+    }
     cnt[4] = cp->chunk_index == 0 ? 1 : 0;  // beta_g2 travels with chunk 0 (aggregation.rs:103-111)
     return SS_OK;
 }
@@ -1073,16 +1027,17 @@ int ss_phase1_decompress(const ss_phase1_params* p, const uint8_t* in, size_t in
     if (!p || !in || !out) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "null argument");
     if (p->proving_system != SS_GROTH16) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "only the Groth16 layout is implemented");
     if (check < 0 || check > 3) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "bad check mode");
-    ss_phase1_sizes z;
-    int rc = phase1_sizes(p, &z);
-    if (rc) return rc;
-    if (in_len < z.contribution_size - z.public_key_size)
-        return fail(SS_ERR_INVALID_LENGTH, 0, z.contribution_size - z.public_key_size, in_len, "compressed buffer too short");
-    if (out_len < z.accumulator_size) return fail(SS_ERR_INVALID_LENGTH, 0, z.accumulator_size, out_len, "output buffer too short");
-    uint64_t io[5], oo[5];
-    vector_offsets(p->curve, z, 1, io);
-    vector_offsets(p->curve, z, 0, oo);
-    const uint64_t cnt[5] = {z.g1_chunk_size, z.other_chunk_size, z.other_chunk_size, z.other_chunk_size, 1};
+    Phase1Layout c, u;
+    int rc;
+    if ((rc = phase1_layout(p, 1, &c)) || (rc = phase1_layout(p, 0, &u))) return rc;
+    if ((rc = check_length(c, in_len, "compressed buffer too short"))) return rc;
+    if ((rc = check_length(u, out_len, "output buffer too short"))) return rc;
+    uint64_t io[5], oo[5], cnt[5];
+    for (int v = 0; v < 5; v++) {
+        io[v] = c.v[v].off;
+        oo[v] = u.v[v].off;
+        cnt[v] = c.v[v].count;
+    }
     return copy_vectors(p->curve, in, io, 1, out, oo, 0, cnt, check);
 }
 
@@ -1093,28 +1048,13 @@ int ss_phase1_sizes_of(const ss_phase1_params* p, ss_phase1_sizes* out) { return
 // on the device (encode_point) and replicated into the caller's buffer; the 64-byte hash prefix is not touched.
 int ss_phase1_initialization(const ss_phase1_params* p, uint8_t* output, size_t output_len, int compressed_output) {
     if (!p || !output) return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "null argument");
-    ss_phase1_sizes z;
-    int rc = phase1_sizes(p, &z);
+    Phase1Layout L;  // split_mut (buffers.rs:246-288)
+    int rc = phase1_layout(p, compressed_output, &L);
     if (rc) return rc;
-    const GroupOps* gs[2] = {group_ops(p->curve, SS_G1), group_ops(p->curve, SS_G2)};
-    const uint64_t s1 = compressed_output ? gs[0]->csize : gs[0]->usize, s2 = compressed_output ? gs[1]->csize : gs[1]->usize;
-    // split_mut (buffers.rs:246-288): Groth16 = [tau_g1][tau_g2][alpha_g1][beta_g1][beta_g2]; Marlin = [tau_g1] and, in the
-    // buffer of chunk 0, [tau_g2 x (k+2)][alpha_g1 x (3+3k)] — no beta_g1 / beta_g2 slots at all.
-    const bool marlin = p->proving_system == SS_MARLIN;
-    if (!marlin && p->proving_system != SS_GROTH16)
+    const GroupOps* gs[2] = {L.v[0].ops, L.v[1].ops};
+    if (p->proving_system != SS_MARLIN && p->proving_system != SS_GROTH16)
         return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "unknown proving system %d", p->proving_system);
-    const uint64_t mk = p->total_size_in_log2;
-    const uint64_t cnt[5] = {z.g1_chunk_size,
-                             marlin ? (is_chunk0(p) ? mk + 2 : 0) : z.other_chunk_size,
-                             marlin ? (is_chunk0(p) ? 3 + 3 * mk : 0) : z.other_chunk_size,
-                             marlin ? 0 : z.other_chunk_size,
-                             marlin ? 0u : 1u};
-    const int grp[5] = {0, 1, 0, 0, 1};
-    uint64_t off[6];
-    off[0] = 64;
-    for (int v = 0; v < 5; v++) off[v + 1] = off[v] + cnt[v] * (grp[v] ? s2 : s1);
-    const uint64_t need = off[5];
-    if (output_len < need) return fail(SS_ERR_INVALID_LENGTH, 0, need, output_len, "output buffer too short");
+    if ((rc = check_length(L, output_len, "output buffer too short"))) return rc;
     if (!gs[0]->has_generator || !gs[1]->has_generator)
         return fail(SS_ERR_INVALID_ARGUMENT, 0, 0, 0, "the reference's generator constant of %s is not known to this build",
                     gs[0]->has_generator ? gs[1]->name : gs[0]->name);
@@ -1125,7 +1065,8 @@ int ss_phase1_initialization(const ss_phase1_params* p, uint8_t* output, size_t 
     for (int g = 0; g < 2; g++) {
         gs[g]->generator(reinterpret_cast<uint32_t*>(lg.l->buf) + g * 256, compressed_output, lg.l->stream);
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(gen[g], lg.l->buf + g * 1024, g ? s2 : s1, cudaMemcpyDeviceToHost, lg.l->stream));
+        CU(cudaMemcpyAsync(gen[g], lg.l->buf + g * 1024, compressed_output ? gs[g]->csize : gs[g]->usize,
+                           cudaMemcpyDeviceToHost, lg.l->stream));
     }
     CU(cudaStreamSynchronize(lg.l->stream));
     auto fill = [&](uint8_t* dst, const uint8_t* el, uint64_t sz, uint64_t count) {
@@ -1137,7 +1078,7 @@ int ss_phase1_initialization(const ss_phase1_params* p, uint8_t* output, size_t 
             done += k;
         }
     };
-    for (int v = 0; v < 5; v++) fill(output + off[v], gen[grp[v]], grp[v] ? s2 : s1, cnt[v]);
+    for (const Phase1Layout::Vector& e : L.v) fill(output + e.off, gen[e.group], e.size, e.count);
     return SS_OK;
 }
 

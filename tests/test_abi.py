@@ -9,8 +9,11 @@ import pytest
 
 import pyref as R
 import snark_setup_b200 as S
+from snark_setup_b200 import ffi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+SIZE_FIELDS = ("powers_length", "powers_g1_length", "g1_chunk_size", "other_chunk_size", "accumulator_size",
+               "contribution_size", "public_key_size", "hash_size")
 
 
 def _have_gpu():
@@ -39,9 +42,32 @@ def test_sizes_match_reference_formulas():
                                     (4, 8, 1, 3, 8), (5, 7, 1, 2, 20)):
             a = S.Phase1Parameters(cid, k, bs, mode, ci, cs)
             b = R.Phase1Parameters(cv, k, bs, mode, ci, cs)
-            for f in ("powers_length", "powers_g1_length", "g1_chunk_size", "other_chunk_size", "accumulator_size",
-                      "contribution_size", "public_key_size", "hash_size"):
+            for f in SIZE_FIELDS:
                 assert getattr(a, f) == getattr(b, f), (cv.name, k, mode, ci, f)
+        # Marlin: tau_g1 over 2^k powers, plus k+2 tau_g2 and 3+3k alpha_g1 elements in the buffer of chunk 0 only
+        for k, bs, mode, ci, cs in ((3, 8, 0, 0, 0), (3, 8, 1, 0, 4), (3, 8, 1, 1, 4), (4, 8, 1, 3, 4), (5, 7, 1, 2, 12),
+                                    (10, 256, 0, 0, 0)):
+            a = S.Phase1Parameters(cid, k, bs, mode, ci, cs, 1)
+            b = R.Phase1Parameters(cv, k, bs, mode, ci, cs, R.MARLIN)
+            for f in SIZE_FIELDS:
+                assert getattr(a, f) == getattr(b, f), (cv.name, "marlin", k, mode, ci, f)
+    with pytest.raises(ffi.InvalidChunk):  # a Marlin chunk must start below 2^power
+        S.Phase1Parameters(S.BLS12_377, 3, 8, 1, 2, 4, 1)
+
+
+def test_relayout_length_errors_without_device():
+    """decompress / split / aggregation check their buffers against the layout before any device call."""
+    full = S.Phase1Parameters(S.BLS12_377, 3, 8)
+    chunk = S.Phase1Parameters(S.BLS12_377, 3, 8, 1, 1, 4)
+    with pytest.raises(S.InvalidLength) as ei:  # compressed full accumulator
+        S.phase1_decompress(full, bytes(100))
+    assert (ei.value.expected, ei.value.got) == (2416, 100)
+    with pytest.raises(S.InvalidLength) as ei:  # uncompressed full accumulator
+        S.phase1_split_chunk(chunk, bytes(100), False, False)
+    assert (ei.value.expected, ei.value.got) == (4768, 100)
+    with pytest.raises(S.InvalidLength) as ei:  # compressed chunk 1 of size 4
+        S.phase1_aggregate_chunk(chunk, bytes(10), True, bytearray(full.get_length(False)), False)
+    assert (ei.value.expected, ei.value.got) == (1120, 10)
 
 
 def test_argument_errors_are_reported_without_device():
