@@ -42,7 +42,7 @@ extern "C" {
  * ss_groth16_params_*, ss_qap_dot_product) — without endomorphism speed-ups.  Their radix-2 domains reach 2^30 (MNT4-753
  * Fr) and 2^15 (MNT6-753 Fr); a larger domain fails with SS_ERR_INVALID_ARGUMENT.  Not available for them:
  * ss_phase1_initialization (the arkworks G2 generator constants are not known to this build) and the device pairing
- * checks (ss_*same_ratio*; the (s, sx) pairs are returned for the host's check_same_ratio as SURVEY.md §8 A12 places
+ * checks (ss_*same_ratio*, ss_phase2_check_ratio_pairs, ss_phase2_verification; the (s, sx) pairs are returned for the host's check_same_ratio as SURVEY.md §8 A12 places
  * it). */
 typedef enum { SS_CURVE_BLS12_377 = 0, SS_CURVE_BW6_761 = 1, SS_CURVE_MNT4_753 = 2, SS_CURVE_MNT6_753 = 3 } ss_curve;
 typedef enum { SS_G1 = 0, SS_G2 = 1 } ss_group;
@@ -371,6 +371,68 @@ int ss_phase1_check_ratio_pairs(int curve, const uint8_t* pairs, const uint8_t* 
 int ss_qap_dot_product(int curve, int group, const uint8_t* bases, int bases_compressed, int check, size_t n_bases,
                        const uint64_t* row_ptr, const uint32_t* index, const uint8_t* coeffs, size_t rows, uint8_t* out,
                        int out_compressed);
+
+/* -------------------------------------------------------------------------------------------- */
+/* phase 2: MPCParameters::contribute / verify on the H and L queries (SURVEY.md config C5)      */
+/* -------------------------------------------------------------------------------------------- */
+/* MPCParameters::contribute, hot half — phase2/src/parameters.rs:286-307 (streaming twin
+ * phase2/src/chunked_groth16.rs:237,387-466): every element of h_query (n_h) and l_query (n_l) <- delta^-1 * element,
+ * IN PLACE, read with `check` and re-written with the same `compressed`; delta_g1 (one G1 element) and delta_g2 (one G2
+ * element) <- delta * element, in place, serialized and read the same way (either may be NULL).  delta = canonical
+ * scalar; 0 or >= r => SS_ERR_INVALID_ARGUMENT.  delta^-1 is computed on the device.  Bases read with No /
+ * OnlyNonZero follow ss_set_strict_unchecked_inputs.  A failing element is reported with its query-relative index and
+ * the query's name ("h_query" / "l_query"); the H query is reported when both fail.  The two queries run concurrently
+ * unless ss_set_concurrent_vectors(0); results are identical either way.  Parsing the parameters file, the
+ * contribution's public key and the transcript hash stay with the caller. */
+int ss_phase2_contribute(int curve, const uint8_t* delta, uint8_t* h_query, size_t n_h, uint8_t* l_query, size_t n_l,
+                         int compressed, int check, uint8_t* delta_g1, uint8_t* delta_g2);
+
+/* Shard `shard_index` of `shard_count` of the same call: each query is cut into shard_count equal contiguous parts
+ * (see ss_phase1_computation_shard); h_query / l_query are the WHOLE queries and only the shard's byte ranges are read
+ * and written.  delta_g1 / delta_g2 belong to shard 0.  With several devices selected in ss_init the shard is divided
+ * once more among them. */
+int ss_phase2_contribute_shard(int curve, const uint8_t* delta, uint8_t* h_query, size_t n_h, uint8_t* l_query,
+                               size_t n_l, int compressed, int check, uint8_t* delta_g1, uint8_t* delta_g2,
+                               uint32_t shard_index, uint32_t shard_count);
+
+/* The H / L half of MPCParameters::verify — phase2/src/parameters.rs:393-407 (chunked_check_ratio,
+ * chunked_groth16.rs:521-566): merge_pairs(before.h, after.h) and merge_pairs(before.l, after.l) of the shard's part of
+ * the queries.  `pairs` <- s_h || sx_h || s_l || sx_l, uncompressed G1 (s = sum rho_i before_i, sx = sum rho_i after_i),
+ * rho_i from rho_seed and the global element index as in ss_merge_pairs, so the partial pairs of any sharding add up
+ * (ss_phase2_reduce_partial_pairs) to the whole-query pairs byte for byte.  `before` is decoded with check_before and
+ * `after` with check_after (CheckForCorrectness, as in ss_transcode).  Unless subgroup_mode == SS_SUBGROUP_NO every
+ * element of `after` must also satisfy r*P = O, else SS_ERR_INCORRECT_SUBGROUP (read_groth16_fast's
+ * check_subgroup_membership, parameters.rs:566-581); `before`, checked in its own round, gets no subgroup pass.  An
+ * empty whole query => SS_ERR_BATCH_TOO_SMALL; an empty part leaves identities.  Errors name the query and give its
+ * query-relative index (H before L). */
+int ss_phase2_verification_pairs(int curve, const uint8_t* h_before, const uint8_t* h_after, size_t n_h,
+                                 const uint8_t* l_before, const uint8_t* l_after, size_t n_l, int compressed,
+                                 int check_before, int check_after, int subgroup_mode, const uint8_t* rho_seed,
+                                 uint8_t* pairs, uint32_t shard_index, uint32_t shard_count);
+
+/* Bytes of a phase-2 `pairs` blob (4 * G1 uncompressed), and the element-wise group sums of `count` partial blobs laid
+ * out back to back (see ss_phase1_reduce_partial_pairs). */
+size_t ss_phase2_pairs_size(int curve);
+int ss_phase2_reduce_partial_pairs(int curve, const uint8_t* partials, int count, uint8_t* pairs);
+
+/* The verdict of MPCParameters::verify's ratio checks from `pairs` (whole-query or reduced) and the uncompressed delta
+ * elements, three check_same_ratio (setup-utils/src/helpers.rs:410-424) in ONE launch.  SS_ERR_INVALID_RATIO with
+ * ss_last_error().index = the lowest failing check:
+ *   0 = delta: same_ratio((G1, delta_g1_after), (G2, delta_g2_after)) with arkworks' generators — the reference's
+ *       "delta consistent in G2" check, restated from memory of parameters.rs:314-411, not checked against it;
+ *   1 = H, 2 = L: same_ratio(merge_pairs(before, after), (delta_g2_after, delta_g2_before)), parameters.rs:393-407.
+ * MNT4-753 / MNT6-753 have no device pairing => SS_ERR_INVALID_ARGUMENT.  The byte comparisons of the unchanged parts,
+ * pubkey.delta_after == delta_g1 and the transcript / proof-of-knowledge checks (hash_to_g2) stay with the caller. */
+int ss_phase2_check_ratio_pairs(int curve, const uint8_t* pairs, const uint8_t* delta_g1_after,
+                                const uint8_t* delta_g2_before, const uint8_t* delta_g2_after);
+
+/* ss_phase2_verification_pairs over the whole queries followed by ss_phase2_check_ratio_pairs.  The delta elements are
+ * serialized with `compressed`; delta_g2_before is read with check_before, the two `after` elements with check_after.
+ * MNT4-753 / MNT6-753 => SS_ERR_INVALID_ARGUMENT before any query is read. */
+int ss_phase2_verification(int curve, const uint8_t* h_before, const uint8_t* h_after, size_t n_h,
+                           const uint8_t* l_before, const uint8_t* l_after, size_t n_l, int compressed,
+                           int check_before, int check_after, int subgroup_mode, const uint8_t* delta_g1_after,
+                           const uint8_t* delta_g2_before, const uint8_t* delta_g2_after, const uint8_t* rho_seed);
 
 #ifdef __cplusplus
 }

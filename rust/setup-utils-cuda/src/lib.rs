@@ -7,7 +7,8 @@
 //! (phase1/src/computation.rs:16-25) and the per-vector half of `Phase1::verification`
 //! (phase1/src/verification.rs:26-40,217-411) become one call each; further down the SURVEY §8f rows: verdicts from
 //! ratio pairs, accumulator re-layout (`Phase1::aggregation` / `split` / `decompress`), `Groth16Params::new`, group
-//! IFFT / H query and the QAP row sums of phase 2.
+//! IFFT / H query and the QAP row sums of phase 2, and phase 2's `MPCParameters::contribute` / `verify` on the H and L
+//! queries (`phase2_contribute`, `phase2_verify`, sharded through `phase2_verification_pairs`).
 //!
 //! The seam is at byte-slice granularity: arkworks' `Affine<P>` is not `repr(C)`, so the generic in-memory entry
 //! points serialise to the canonical uncompressed form, call the engine, and read the result back; the phase1
@@ -774,4 +775,152 @@ pub fn qap_dot_product<C: CudaGroup>(
         )
     })?;
     Ok(read_points::<C>(&out, rows))
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// phase 2: MPCParameters::contribute / verify on the H and L queries (SURVEY.md config C5)
+// ------------------------------------------------------------------------------------------------------------------
+
+fn g1_size<E: CudaCurve>(compression: UseCompression) -> usize {
+    match compression {
+        Compress::Yes => E::G1Affine::zero().compressed_size(),
+        Compress::No => E::G1Affine::zero().uncompressed_size(),
+    }
+}
+
+/// The hot half of `MPCParameters::contribute` (phase2/src/parameters.rs:286-307; streaming twin
+/// chunked_groth16.rs:387-466): every element of the serialized `h_query` / `l_query` <- delta^-1 * element and
+/// `delta_g1` / `delta_g2` <- delta * element, in place, all serialized with `compression` and read with
+/// `check_input_for_correctness`.  `shard = (index, count)` processes that index-range part of each query only
+/// (`(0, 1)`: whole queries); delta_g1 / delta_g2 belong to shard 0.
+pub fn phase2_contribute<E: CudaCurve>(
+    h_query: &mut [u8],
+    l_query: &mut [u8],
+    delta_g1: Option<&mut [u8]>,
+    delta_g2: Option<&mut [u8]>,
+    delta: &E::ScalarField,
+    compression: UseCompression,
+    check_input_for_correctness: CheckForCorrectness,
+    shard: (u32, u32),
+) -> Result<()> {
+    let size = g1_size::<E>(compression);
+    let d = scalar_bytes(delta);
+    let p1 = delta_g1.map_or(core::ptr::null_mut(), |b| b.as_mut_ptr());
+    let p2 = delta_g2.map_or(core::ptr::null_mut(), |b| b.as_mut_ptr());
+    check(unsafe {
+        ffi::ss_phase2_contribute_shard(
+            E::CURVE_ID,
+            d.as_ptr(),
+            h_query.as_mut_ptr(),
+            h_query.len() / size,
+            l_query.as_mut_ptr(),
+            l_query.len() / size,
+            flag(compression),
+            check_mode(check_input_for_correctness),
+            p1,
+            p2,
+            shard.0,
+            shard.1,
+        )
+    })
+}
+
+/// `merge_pairs(before.h, after.h)` and `merge_pairs(before.l, after.l)` of MPCParameters::verify
+/// (phase2/src/parameters.rs:393-407) over shard `shard` of the serialized queries, with read_groth16_fast's subgroup
+/// check on `after` (:566-581): the pairs blob (s_h, sx_h, s_l, sx_l), partial sums for a shard.
+pub fn phase2_verification_pairs<E: CudaCurve>(
+    before: (&[u8], &[u8]),
+    after: (&[u8], &[u8]),
+    compression: UseCompression,
+    check_before: CheckForCorrectness,
+    check_after: CheckForCorrectness,
+    subgroup_check_mode: SubgroupCheckMode,
+    shard: (u32, u32),
+) -> Result<Vec<u8>> {
+    let size = g1_size::<E>(compression);
+    assert!(before.0.len() == after.0.len() && before.1.len() == after.1.len());
+    let seed = rho_seed();
+    let mut pairs = vec![0u8; unsafe { ffi::ss_phase2_pairs_size(E::CURVE_ID) }];
+    check(unsafe {
+        ffi::ss_phase2_verification_pairs(
+            E::CURVE_ID,
+            before.0.as_ptr(),
+            after.0.as_ptr(),
+            before.0.len() / size,
+            before.1.as_ptr(),
+            after.1.as_ptr(),
+            before.1.len() / size,
+            flag(compression),
+            check_mode(check_before),
+            check_mode(check_after),
+            subgroup_mode(subgroup_check_mode),
+            seed.as_ptr(),
+            pairs.as_mut_ptr(),
+            shard.0,
+            shard.1,
+        )
+    })?;
+    Ok(pairs)
+}
+
+/// Element-wise sums of the shards' phase-2 pairs blobs.
+pub fn phase2_reduce_partial_pairs<E: CudaCurve>(blobs: &[Vec<u8>]) -> Result<Vec<u8>> {
+    let size = unsafe { ffi::ss_phase2_pairs_size(E::CURVE_ID) };
+    assert!(blobs.iter().all(|b| b.len() == size));
+    let all: Vec<u8> = blobs.concat();
+    let mut pairs = vec![0u8; size];
+    check(unsafe { ffi::ss_phase2_reduce_partial_pairs(E::CURVE_ID, all.as_ptr(), blobs.len() as c_int, pairs.as_mut_ptr()) })?;
+    Ok(pairs)
+}
+
+/// The ratio checks of MPCParameters::verify from a (reduced) pairs blob, on the device: 0 = delta_g1 / delta_g2
+/// consistency, 1 = H, 2 = L (parameters.rs:393-407) — `ss_last_error().index` names the failing one.
+pub fn phase2_check_ratio_pairs<E: CudaCurve>(
+    pairs_blob: &[u8],
+    delta_g1_after: &E::G1Affine,
+    delta_g2_before: &E::G2Affine,
+    delta_g2_after: &E::G2Affine,
+) -> Result<()> {
+    assert_eq!(pairs_blob.len(), unsafe { ffi::ss_phase2_pairs_size(E::CURVE_ID) });
+    let d1 = points_bytes(&[*delta_g1_after]);
+    let (d2b, d2a) = (points_bytes(&[*delta_g2_before]), points_bytes(&[*delta_g2_after]));
+    check(unsafe { ffi::ss_phase2_check_ratio_pairs(E::CURVE_ID, pairs_blob.as_ptr(), d1.as_ptr(), d2b.as_ptr(), d2a.as_ptr()) })
+}
+
+/// The H / L queries and delta checks of MPCParameters::verify (phase2/src/parameters.rs:314-411) in one call: queries
+/// and the three delta elements serialized with `compression`.  The byte comparisons of the unchanged parts and the
+/// proof-of-knowledge / transcript checks stay with the caller.
+pub fn phase2_verify<E: CudaCurve>(
+    before: (&[u8], &[u8]),
+    after: (&[u8], &[u8]),
+    delta_g1_after: &[u8],
+    delta_g2_before: &[u8],
+    delta_g2_after: &[u8],
+    compression: UseCompression,
+    check_before: CheckForCorrectness,
+    check_after: CheckForCorrectness,
+    subgroup_check_mode: SubgroupCheckMode,
+) -> Result<()> {
+    let size = g1_size::<E>(compression);
+    assert!(before.0.len() == after.0.len() && before.1.len() == after.1.len());
+    let seed = rho_seed();
+    check(unsafe {
+        ffi::ss_phase2_verification(
+            E::CURVE_ID,
+            before.0.as_ptr(),
+            after.0.as_ptr(),
+            before.0.len() / size,
+            before.1.as_ptr(),
+            after.1.as_ptr(),
+            before.1.len() / size,
+            flag(compression),
+            check_mode(check_before),
+            check_mode(check_after),
+            subgroup_mode(subgroup_check_mode),
+            delta_g1_after.as_ptr(),
+            delta_g2_before.as_ptr(),
+            delta_g2_after.as_ptr(),
+            seed.as_ptr(),
+        )
+    })
 }

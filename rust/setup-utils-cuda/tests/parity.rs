@@ -166,3 +166,93 @@ fn cuda_sharded_verification_and_relayout() {
     setup_utils_cuda::phase1_decompress(&response[..n_resp], &mut got, CheckForCorrectness::No, &params).unwrap();
     assert_eq!(want[64..], got[64..]);
 }
+
+/// Phase 2: `MPCParameters::contribute` updates delta_g1 / delta_g2 by delta and the H and L queries by delta^-1
+/// (phase2/src/parameters.rs:286-307), and `verify` checks them with merge_pairs + same_ratio (:393-407).  Building
+/// MPCParameters needs a circuit, so the reference side here is that body through setup_utils (batch_mul, merge_pairs,
+/// same_ratio) on compressed query bytes; the engine side is one call each way, whole and as three shards.
+#[test]
+fn cuda_phase2_contribute_and_verify_match_setup_utils() {
+    use ark_bls12_377::{Fr, G1Affine, G2Affine};
+    use ark_ec::{AffineRepr, CurveGroup};
+    use ark_ff::{Field, UniformRand};
+    use ark_serialize::{CanonicalDeserialize, CanonicalSerialize};
+    let mut rng = derive_rng_from_seed(b"parity-5");
+    let (nh, nl) = (255, 256);
+    let pts = |n: usize, rng: &mut _| -> Vec<G1Affine> { (0..n).map(|_| (G1Affine::generator() * Fr::rand(rng)).into_affine()).collect() };
+    let (h, l) = (pts(nh, &mut rng), pts(nl, &mut rng));
+    let ser = |v: &[G1Affine]| -> Vec<u8> {
+        let mut b = Vec::new();
+        for p in v {
+            p.serialize_compressed(&mut b).unwrap();
+        }
+        b
+    };
+    let delta = Fr::rand(&mut rng);
+    let d1_before = (G1Affine::generator() * Fr::rand(&mut rng)).into_affine();
+    let d2_before = (G2Affine::generator() * Fr::rand(&mut rng)).into_affine();
+
+    // reference body: delta_g1 *= delta, delta_g2 *= delta, queries batch_mul'd by delta^-1
+    let (mut h_ref, mut l_ref) = (h.clone(), l.clone());
+    let inv = delta.inverse().unwrap();
+    setup_utils::batch_mul(&mut h_ref, &inv, BatchExpMode::Auto).unwrap();
+    setup_utils::batch_mul(&mut l_ref, &inv, BatchExpMode::Auto).unwrap();
+    let d1_after = (d1_before * delta).into_affine();
+    let d2_after = (d2_before * delta).into_affine();
+
+    let (mut hb, mut lb) = (ser(&h), ser(&l));
+    let mut d1b = ser(&[d1_before]);
+    let mut d2b = Vec::new();
+    d2_before.serialize_compressed(&mut d2b).unwrap();
+    let d2_before_bytes = d2b.clone();
+    setup_utils_cuda::phase2_contribute::<Bls12_377>(
+        &mut hb, &mut lb, Some(&mut d1b), Some(&mut d2b), &delta, UseCompression::Yes, CheckForCorrectness::Full, (0, 1),
+    )
+    .unwrap();
+    assert_eq!(hb, ser(&h_ref));
+    assert_eq!(lb, ser(&l_ref));
+    assert_eq!(G1Affine::deserialize_compressed(&d1b[..]).unwrap(), d1_after);
+    assert_eq!(G2Affine::deserialize_compressed(&d2b[..]).unwrap(), d2_after);
+
+    // three shards into one pair of buffers give the same bytes
+    let (mut hs, mut ls) = (ser(&h), ser(&l));
+    for s in 0..3u32 {
+        setup_utils_cuda::phase2_contribute::<Bls12_377>(&mut hs, &mut ls, None, None, &delta, UseCompression::Yes, CheckForCorrectness::No, (s, 3))
+            .unwrap();
+    }
+    assert_eq!((hs, ls), (hb.clone(), lb.clone()));
+
+    // verify: the reference's verdict on the engine's output, and the engine's verdict
+    let g2_pair = (d2_after, d2_before);
+    assert!(same_ratio::<Bls12_377>(&setup_utils::merge_pairs(&h, &h_ref), &g2_pair));
+    assert!(same_ratio::<Bls12_377>(&setup_utils::merge_pairs(&l, &l_ref), &g2_pair));
+    let (h0, l0) = (ser(&h), ser(&l));
+    setup_utils_cuda::phase2_verify::<Bls12_377>(
+        (&h0, &l0), (&hb, &lb), &d1b, &d2_before_bytes, &d2b, UseCompression::Yes, CheckForCorrectness::No,
+        CheckForCorrectness::OnlyNonZero, SubgroupCheckMode::Auto,
+    )
+    .unwrap();
+    let blobs: Vec<Vec<u8>> = (0..3u32)
+        .map(|s| {
+            setup_utils_cuda::phase2_verification_pairs::<Bls12_377>(
+                (&h0, &l0), (&hb, &lb), UseCompression::Yes, CheckForCorrectness::No, CheckForCorrectness::OnlyNonZero,
+                SubgroupCheckMode::Auto, (s, 3),
+            )
+            .unwrap()
+        })
+        .collect();
+    let pairs = setup_utils_cuda::phase2_reduce_partial_pairs::<Bls12_377>(&blobs).unwrap();
+    setup_utils_cuda::phase2_check_ratio_pairs::<Bls12_377>(&pairs, &d1_after, &d2_before, &d2_after).unwrap();
+    // an H element replaced by its neighbour is rejected by both
+    let g1c = 48;
+    let mut bad = hb.clone();
+    bad.copy_within(g1c..2 * g1c, 0);
+    assert!(setup_utils_cuda::phase2_verify::<Bls12_377>(
+        (&h0, &l0), (&bad, &lb), &d1b, &d2_before_bytes, &d2b, UseCompression::Yes, CheckForCorrectness::No,
+        CheckForCorrectness::OnlyNonZero, SubgroupCheckMode::Auto,
+    )
+    .is_err());
+    let mut h_bad = h_ref.clone();
+    h_bad[0] = h_bad[1];
+    assert!(!same_ratio::<Bls12_377>(&setup_utils::merge_pairs(&h, &h_bad), &g2_pair));
+}

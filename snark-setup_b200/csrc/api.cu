@@ -627,10 +627,11 @@ int check_length(const Phase1Layout& L, uint64_t len, const char* what) {
 
 // The (s, sx) pairs blob of the four ratio-checked vectors: slot v holds s || sx of vector v, uncompressed, so
 // 4 x (s || sx) in the order G1, G2, G1, G1.  pair_slot(curve, 4) is the size of the blob, 0 for an unknown curve.
-size_t pair_slot(int curve, int v) {
+// `groups` gives the slots of another blob (phase 2: the H and L queries, both G1).
+size_t pair_slot(int curve, int v, const int* groups = kVecGroup) {
     size_t off = 0;
     for (int u = 0; u < v; u++) {
-        const GroupOps* o = group_ops(curve, kVecGroup[u]);
+        const GroupOps* o = group_ops(curve, groups[u]);
         if (!o) return 0;
         off += 2 * (size_t)o->usize;
     }
@@ -1163,3 +1164,4 @@ int ss_phase1_computation_shard_dev(const ss_phase1_params* p, const void* d_inp
 #include "api_fft.inl"
 #include "api_pairing.inl"
 #include "api_qap.inl"
+#include "api_phase2.inl"

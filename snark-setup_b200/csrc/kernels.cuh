@@ -750,4 +750,7 @@ const GroupOps& ops_mnt4_g2();
 const GroupOps& ops_mnt6_g1();
 const GroupOps& ops_mnt6_g2();
 
+// out = a^-1 in the scalar field of curve `curve` (ss_curve), Montgomery in and out; kern_fr.cu
+void fr_inverse(int curve, const uint32_t* a_mont, uint32_t* out_mont, cudaStream_t s);
+
 }  // namespace ss

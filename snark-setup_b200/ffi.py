@@ -595,3 +595,91 @@ def phase1_computation_dev(params: Phase1Parameters, d_in, in_len, d_out, out_le
                   C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint32, C.c_void_p]
     _check(f(C.byref(params.c), d_in, in_len, d_out, out_len, int(compressed_input), int(compressed_output),
              check_input, _scalar(cv, tau), _scalar(cv, alpha), _scalar(cv, beta), si, sc, stream))
+
+
+# ---- phase 2: MPCParameters::contribute / verify on the H and L queries -----------------------------------------------
+def phase2_pairs_size(curve):
+    f = lib().ss_phase2_pairs_size
+    f.restype = C.c_size_t
+    return f(curve)
+
+
+def _split_phase2_pairs(curve, raw):
+    u = element_size(curve, G1, False)
+    return [(raw[0:u], raw[u:2 * u]), (raw[2 * u:3 * u], raw[3 * u:4 * u])]
+
+
+def phase2_contribute(curve, delta, h_query: bytearray, l_query: bytearray, compressed, check=CHECK_NO, delta_g1=None,
+                      delta_g2=None, shard=None):
+    """The hot half of MPCParameters::contribute (phase2/src/parameters.rs:286-307): h_query / l_query <- delta^-1 * each
+    element and delta_g1 / delta_g2 <- delta * element, all serialized with `compressed` and updated IN PLACE
+    (bytearrays; delta_g1 / delta_g2 may be None).  shard=(index, count): only that index-range shard of each query."""
+    sz = element_size(curve, G1, compressed)
+    nh, nl = len(h_query) // sz, len(l_query) // sz
+    ph, k1 = _buf(h_query) if nh else (None, None)
+    pl, k2 = _buf(l_query) if nl else (None, None)
+    pd1, k3 = _buf(delta_g1) if delta_g1 is not None else (None, None)
+    pd2, k4 = _buf(delta_g2) if delta_g2 is not None else (None, None)
+    si, sc = shard if shard is not None else (0, 1)
+    f = lib().ss_phase2_contribute_shard
+    f.argtypes = [C.c_int, C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p,
+                  C.c_void_p, C.c_uint32, C.c_uint32]
+    _check(f(curve, _scalar(curve, delta), ph, nh, pl, nl, int(bool(compressed)), check, pd1, pd2, si, sc))
+
+
+def phase2_verification_pairs(curve, h_before, h_after, l_before, l_after, compressed, check_before=CHECK_NO,
+                              check_after=CHECK_ONLY_NON_ZERO, subgroup_mode=SUBGROUP_AUTO, seed=None, shard=None,
+                              raw=False):
+    """merge_pairs(before, after) of the H and L queries (phase2/src/parameters.rs:393-407) ->
+    [(s_h, sx_h), (s_l, sx_l)] uncompressed, or the raw blob; shard=(index, count) gives that shard's partial sums."""
+    sz = element_size(curve, G1, compressed)
+    nh, nl = len(h_before) // sz, len(l_before) // sz
+    if len(h_after) // sz != nh or len(l_after) // sz != nl:
+        raise InvalidLength("before / after lengths differ", 0, nh, len(h_after) // sz)
+    pairs = C.create_string_buffer(phase2_pairs_size(curve))
+    bufs = [_buf(b) if len(b) else (None, None) for b in (h_before, h_after, l_before, l_after)]
+    si, sc = shard if shard is not None else (0, 1)
+    f = lib().ss_phase2_verification_pairs
+    f.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int,
+                  C.c_int, C.c_int, C.c_char_p, C.c_void_p, C.c_uint32, C.c_uint32]
+    _check(f(curve, bufs[0][0], bufs[1][0], nh, bufs[2][0], bufs[3][0], nl, int(bool(compressed)), check_before,
+             check_after, subgroup_mode, bytes(seed) if seed is not None else None, pairs, si, sc))
+    return pairs.raw if raw else _split_phase2_pairs(curve, pairs.raw)
+
+
+def phase2_reduce_partial_pairs(curve, blobs, raw=False):
+    """Element-wise group sums of the shards' partial phase-2 pairs blobs."""
+    n = phase2_pairs_size(curve)
+    blobs = [bytes(b) for b in blobs]
+    assert all(len(b) == n for b in blobs)
+    out = C.create_string_buffer(n)
+    f = lib().ss_phase2_reduce_partial_pairs
+    f.argtypes = [C.c_int, C.c_char_p, C.c_int, C.c_void_p]
+    _check(f(curve, b"".join(blobs), len(blobs), out))
+    return out.raw if raw else _split_phase2_pairs(curve, out.raw)
+
+
+def phase2_check_ratio_pairs(curve, pairs, delta_g1_after, delta_g2_before, delta_g2_after):
+    """The three ratio checks of MPCParameters::verify from a pairs blob and uncompressed delta elements; raises
+    InvalidRatio with .index 0 (delta), 1 (H) or 2 (L)."""
+    f = lib().ss_phase2_check_ratio_pairs
+    f.argtypes = [C.c_int, C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p]
+    _check(f(curve, bytes(pairs), bytes(delta_g1_after), bytes(delta_g2_before), bytes(delta_g2_after)))
+
+
+def phase2_verification(curve, h_before, h_after, l_before, l_after, compressed, delta_g1_after, delta_g2_before,
+                        delta_g2_after, check_before=CHECK_NO, check_after=CHECK_ONLY_NON_ZERO,
+                        subgroup_mode=SUBGROUP_AUTO, seed=None):
+    """phase2_verification_pairs over the whole queries + phase2_check_ratio_pairs; the delta elements are serialized
+    with `compressed`."""
+    sz = element_size(curve, G1, compressed)
+    nh, nl = len(h_before) // sz, len(l_before) // sz
+    if len(h_after) // sz != nh or len(l_after) // sz != nl:
+        raise InvalidLength("before / after lengths differ", 0, nh, len(h_after) // sz)
+    bufs = [_buf(b) if len(b) else (None, None) for b in (h_before, h_after, l_before, l_after)]
+    f = lib().ss_phase2_verification
+    f.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int,
+                  C.c_int, C.c_int, C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p]
+    _check(f(curve, bufs[0][0], bufs[1][0], nh, bufs[2][0], bufs[3][0], nl, int(bool(compressed)), check_before,
+             check_after, subgroup_mode, bytes(delta_g1_after), bytes(delta_g2_before), bytes(delta_g2_after),
+             bytes(seed) if seed is not None else None))
